@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- throughput of the B200 cuboid-proposal hot path (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c3|c2|c4|c5]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c3|c2|c4|c5] [--dump-outputs DIR]
 
 A "step" is one pass of the north-star path over one batch of synthetic frames: line segments detected on the device
 (line_lbd_detect::detect_filter_lines, LSD flavour -- what object_slam sets, main_obj.cpp:365), then detect_cuboid over
@@ -332,6 +332,18 @@ class Mode(object):
                 cx.upload_online(wl["imgs"], wl["Ts"], wl["boxes"], self.lp, self.params)
 
 
+def dump_outputs(out_dir, cx):
+    """--dump-outputs: what a caller of the timed path receives for the batch of its last step (cs_batch_fetch): the top-K cuboid records
+    of every object, one float64 array per record field (objects x K [x field shape]; slots past an object's count are zero), and the
+    count of each object."""
+    recs, counts = cx.fetch()
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "counts.npy"), counts.astype(np.float64))
+    for name in recs.dtype.names:
+        if name != "pad_":
+            np.save(os.path.join(out_dir, "cuboid_%s.npy" % name), recs[name].astype(np.float64))
+
+
 def make_line_params(cs, cx, use_lsd=True):
     det = cs.line_lbd_detect(context=cx)
     det.use_LSD = use_lsd
@@ -533,6 +545,8 @@ def run_ours(args, rank, world, local_rank):
     main_mode = Mode("online_lsd", ctxs, streams, wl, params, line_params(True))
     ms_total, stats, stage_acc = timed(main_mode, args.steps, args.warmup, world > 1)
     sampler.stop_flag = True
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, ctxs[(args.steps - 1) % len(ctxs)])
     my_ms = ms_total
     ms_t = torch.tensor([ms_total], device="cuda", dtype=torch.float64)
     cnt = torch.tensor([stats["n_valid"], stats["n_candidates"], stats["n_frames"], stats["n_objects"]], device="cuda", dtype=torch.float64)
@@ -751,7 +765,11 @@ def main():
     ap.add_argument("--raster-dt", action="store_true", help="A/B: two-pass raster-scan distance transform kernel instead of the cone form")
     ap.add_argument("--seq-lines", action="store_true", help="A/B: the line detectors' sequential kernels (one warp per frame) instead of ordered speculation")
     ap.add_argument("--inflight", type=int, default=24, help="batches in flight on one GPU (contexts driven round-robin)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the cuboid records of the last step's batch (rank 0) "
+                    "to DIR/<name>.npy, float64, for comparing two builds on the same seeded inputs")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the GPU path's outputs (--impl ours)")
     if args.steps is None:
         args.steps = 300 if args.impl == "ours" else 3
     rank = int(os.environ.get("RANK", "0"))

@@ -1,14 +1,16 @@
 """Stage (ii) of the north star, `detect_3d_cuboid::detect_cuboid`, executed by the REFERENCE'S OWN code: detect_3d_cuboid/src/matrix_utils.cpp,
-object_3d_util.cpp and box_proposal_detail.cpp compiled from /root/reference into oracle/_ref/libcuboid_ref.so (oracle/ref/cuboid_ref.cpp;
+object_3d_util.cpp and box_proposal_detail.cpp compiled from the reference's sources into oracle/_ref/libcuboid_ref.so (oracle/ref/cuboid_ref.cpp;
 Eigen replaced by oracle/ref/minieigen.hpp, OpenCV by oracle/ref/minicv.hpp with Canny / distanceTransform / cvtColor forwarded to the
 cv2-pinned restatements) and driven as object_slam/src/main_obj.cpp:354-361,449 drives it.  Every cuboid the reference returns -- which
 proposal wins, its rank among the top k, position, yaw, scale, the 2-D and 3-D corners, both errors, the normalised score, the roll /
 pitch deltas -- must equal the oracle's record, here asserted with ==, not a tolerance (the oracle runs with libm's atan2 for this
 comparison, as the reference does; tests/test_pmath.py ties the arithmetic atan2 the parity tests use to libm's).
 
-Skips where the library was not built (no reference checkout at build time)."""
+What the reference returned is recorded in tests/golden/reference/ (tests/reference_outputs.py), so these tests run without it."""
 import numpy as np
 import pytest
+
+from reference_outputs import Reference, assert_same
 
 FIELDS = ("pos", "rotY", "scale", "box_config_type", "box_corners_2d", "box_corners_3d_world", "rect_detect_2d", "edge_distance_error",
           "edge_angle_error", "normalized_error", "skew_ratio", "down_expand_height", "camera_roll_delta", "camera_pitch_delta")
@@ -18,11 +20,11 @@ MODES = [("default", {}), ("top5", dict(max_cuboid_num=5)), ("roll_pitch", dict(
 
 @pytest.fixture(scope="module")
 def ref(oracle):
-    if not oracle.ref_detect_cuboid_available():
-        pytest.skip("oracle/_ref/libcuboid_ref.so not built (no /root/reference on this machine)")
+    r = Reference(oracle, __name__)
     oracle.lib().orc_set_portable_atan2(0)
-    yield oracle
+    yield r
     oracle.lib().orc_set_portable_atan2(1)
+    r.save()
 
 
 def _same(ref, img, K, T, boxes, lines, p):
@@ -32,10 +34,9 @@ def _same(ref, img, K, T, boxes, lines, p):
     n = 0
     for b in range(len(want)):
         assert len(got[b]) == len(want[b]), b
-        for j in range(len(want[b])):
-            for f in FIELDS:
-                np.testing.assert_array_equal(np.asarray(got[b][j][f], np.float64), np.asarray(want[b][j][f], np.float64), err_msg="%s box %d rank %d" % (f, b, j))
-            n += 1
+        for f in FIELDS:   # every rank of the box at once
+            assert_same(np.asarray(got[b][f], np.float64), want[b][f], err_msg="%s box %d" % (f, b))
+        n += len(want[b])
     return n
 
 

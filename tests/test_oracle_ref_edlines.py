@@ -1,27 +1,28 @@
 """The EDLines oracle (oracle/edl_oracle.cpp) against the REFERENCE'S OWN detector: line_lbd/libs/binary_descriptor.cpp (BinaryDescriptor
-with its nested EDLineDetector) and the reference's headers, compiled from /root/reference into oracle/_ref/libedl_ref.so
+with its nested EDLineDetector) and the reference's headers, compiled from the reference's sources into oracle/_ref/libedl_ref.so
 (oracle/Makefile target `ref`, oracle/ref/edl_ref.cpp + minicv.hpp + fakecv/: the reference files are included from where they lie,
 nothing of them is copied) and driven as line_lbd_detect::detect_raw_lines drives it for use_LSD = false
 (line_lbd/class/line_lbd_allclass.cpp:110-124,165-169).  The key lines of octave 0 must be equal bit for bit, count and order.
 
-The library exists where the reference checkout was present at build time (it travels to the GPU box with the snapshot); without it these
-tests skip, and tests/test_goldens_sequence.py still pins the oracle to the reference through the recorded `edl_raw_checksum_ref`."""
+What the reference returned is recorded in tests/golden/reference/ (tests/reference_outputs.py), so these tests run without it."""
 import numpy as np
 import pytest
+
+from reference_outputs import Reference, assert_same
 
 
 @pytest.fixture(scope="module")
 def ref(oracle):
-    if not oracle.ref_edl_available():
-        pytest.skip("oracle/_ref/libedl_ref.so not built (no /root/reference on this machine)")
-    return oracle
+    r = Reference(oracle, __name__)
+    yield r
+    r.save()
 
 
 def _same(ref, img):
     got = ref.edl_detect(img, 15.0)["raw_lines"]
     want = ref.ref_edl_detect(img)
     assert got.shape == want.shape
-    np.testing.assert_array_equal(got, want)
+    assert_same(got, want)
     return len(want)
 
 

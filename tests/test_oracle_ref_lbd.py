@@ -1,6 +1,7 @@
 """The LBD descriptor / matcher oracle (oracle/lbd_oracle.cpp, SURVEY.md section 8 row f4) against the REFERENCE'S OWN code:
 line_lbd/class/line_lbd_allclass.cpp, libs/binary_descriptor.cpp (computeImpl, computeLBD) and libs/binary_descriptor_matcher.cpp compiled
-from /root/reference into oracle/_ref/liblinelbd_ref.so (oracle/ref/linelbd_ref.cpp: the reference files are included from where they lie).
+from the reference's sources into oracle/_ref/liblinelbd_ref.so (oracle/ref/linelbd_ref.cpp: the reference files are included from where
+they lie).
 
  * detect_descrip_lines(gray, keylines_out, line_descrips) (line_lbd_allclass.cpp:253-272), both detector flavours: the kept key lines --
    end points, angle, lineLength, response, size, numOfPixels -- and their 32-byte descriptors are equal bit for bit, count and order;
@@ -8,17 +9,18 @@ from /root/reference into oracle/_ref/liblinelbd_ref.so (oracle/ref/linelbd_ref.
  * match_line_descrip (:341-356): the same (query, train, distance) triples, including which of several equally near codes the multi-index
    hash meets first.
 
-The library exists where the reference checkout was present at build time (it travels to the GPU box with the snapshot); without it these
-tests skip and tests/golden/expected_lbd.json (written only after this equality held, tools/make_golden_lbd.py) keeps the oracle pinned."""
+What the reference returned is recorded in tests/golden/reference/ (tests/reference_outputs.py), so these tests run without it."""
 import numpy as np
 import pytest
+
+from reference_outputs import Reference, assert_same
 
 
 @pytest.fixture(scope="module")
 def ref(oracle):
-    if not oracle.ref_detect_filter_lines_available():
-        pytest.skip("oracle/_ref/liblinelbd_ref.so not built (no /root/reference on this machine)")
-    return oracle
+    r = Reference(oracle, __name__)
+    yield r
+    r.save()
 
 
 FIELDS = ("sx", "sy", "ex", "ey", "angle", "line_length", "response", "size", "num_pixels")
@@ -29,13 +31,13 @@ def _same_frame(ref, img, use_lsd, thres=15.0):
     ko = ref.lbd_detect_keylines(img, use_lsd, thres)
     assert len(kr) == len(ko)
     for f in FIELDS:
-        np.testing.assert_array_equal(kr[f], ko[f], err_msg=f)
+        assert_same(ko[f], kr[f], err_msg=f)
     do, fo = ref.lbd_compute(img, ko, want_float=True)
-    np.testing.assert_array_equal(do, dr)
+    assert_same(do, dr)
     if len(ko):
         d2, f2 = ref.ref_lbd_compute(img, ko, want_float=True)   # class_id 0 .. n-1, as computeImpl requires
-        np.testing.assert_array_equal(d2, do)
-        np.testing.assert_array_equal(f2, fo)
+        assert_same(do, d2)
+        assert_same(fo, f2)
         assert np.isfinite(fo).all()
     return ko, do
 
@@ -58,7 +60,7 @@ def test_sequence_frames_and_matches_between_neighbours(ref, fixture_b):
             for thres in (25.0, 60.0):
                 a, b = ref.lbd_match(do, prev, thres), ref.ref_match_line_descrip(do, prev, thres)
                 for x, y in zip(a, b):
-                    np.testing.assert_array_equal(x, y)
+                    assert_same(x, y)
         prev = do
     # neighbouring frames of a real sequence (the camera moves a fair way between them): some lines do match
     f0, f1 = fixture_b["frames"][0][0], fixture_b["frames"][1][0]
@@ -77,9 +79,9 @@ def test_octaves_variant_orders_the_ends(ref, fixture_a, use_lsd):
     kz = ref.lbd_order_keylines(ko)
     assert len(kr) == len(kz) and (kz["sx"] != ko["sx"]).any()
     for f in FIELDS:
-        np.testing.assert_array_equal(kr[f], kz[f], err_msg=f)
-    np.testing.assert_array_equal(kr["class_id"], np.arange(len(kr)))
-    np.testing.assert_array_equal(dr, do)                       # descriptors are computed before the swap
+        assert_same(kz[f], kr[f], err_msg=f)
+    assert_same(np.arange(len(kr)), kr["class_id"])
+    assert_same(do, dr)                                         # descriptors are computed before the swap
 
 
 @pytest.mark.parametrize("seed,w,h,kind", [(7, 640, 480, "indoor"), (8, 1242, 375, "kitti")])
@@ -103,8 +105,8 @@ def test_given_keylines_gray_input_and_border_lines(ref):
     kl = ref.lbd_keylines_from_lsd(rows, 160, 120)
     d, f = ref.lbd_compute(img, kl, want_float=True)
     d2, f2 = ref.ref_lbd_compute(img, kl, want_float=True)
-    np.testing.assert_array_equal(d, d2)
-    np.testing.assert_array_equal(f, f2)
+    assert_same(d, d2)
+    assert_same(f, f2)
 
 
 def test_matcher_ties_and_far_codes(ref):
@@ -129,19 +131,19 @@ def test_matcher_ties_and_far_codes(ref):
         t[nt - 1] = t[0]                                   # an exact duplicate: bucket order decides
         for thres in (25.0, 300.0):
             a, b = ref.lbd_match(q, t, thres), ref.ref_match_line_descrip(q, t, thres)
-            np.testing.assert_array_equal(a[0], b[0])
-            np.testing.assert_array_equal(a[2], b[2])
+            assert_same(a[0], b[0])
+            assert_same(a[2], b[2])
             near = a[2] <= 128        # beyond D = 128 the reference never writes results[]: its trainIdx is uninitialised memory, the oracle says -1
-            np.testing.assert_array_equal(a[1][near], b[1][near])
+            assert_same(a[1][near], b[1][near])
             assert (a[1][~near] == -1).all()
     # unrelated codes: distances around 128; every query still gets its nearest code while that is within D = 128
     q = rng.integers(0, 256, (300, 32), dtype=np.uint8)
     t = rng.integers(0, 256, (40, 32), dtype=np.uint8)
     a, b = ref.lbd_match(q, t, 300.0), ref.ref_match_line_descrip(q, t, 300.0)
-    np.testing.assert_array_equal(a[0], b[0])
-    np.testing.assert_array_equal(a[2], b[2])
+    assert_same(a[0], b[0])
+    assert_same(a[2], b[2])
     near = a[2] <= 128
-    np.testing.assert_array_equal(a[1][near], b[1][near])
+    assert_same(a[1][near], b[1][near])
     assert (a[1][~near] == -1).all()
     # the distances themselves are the true minima
     dmin = np.array([[int(np.unpackbits(x ^ y).sum()) for y in t] for x in q]).min(1)

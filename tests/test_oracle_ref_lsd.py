@@ -1,26 +1,27 @@
-"""The LSD oracle (oracle/lsd_oracle.cpp) against the REFERENCE'S OWN lsd.cpp, compiled from /root/reference into
+"""The LSD oracle (oracle/lsd_oracle.cpp) against the REFERENCE'S OWN lsd.cpp, compiled from the reference's sources into
 oracle/_ref/liblsd_ref.so (oracle/Makefile target `ref`, oracle/ref/lsd_ref.cpp + minicv.hpp: the reference file is included from
 where it lies, nothing of it is copied).  Raw segments -- createLineSegmentDetector(LSD_REFINE_ADV)->detect(gray), what
 LSDDetector::detectImpl (line_lbd/libs/LSDDetector.cpp:120-170) gets for octave 0 -- must be equal bit for bit, count and order.
 
-The library exists where the reference checkout was present at build time (it travels to the GPU box with the snapshot); without it these
-tests skip, and tests/test_goldens_sequence.py still pins the oracle to the reference through the recorded `raw_checksum_ref`."""
+What the reference returned is recorded in tests/golden/reference/ (tests/reference_outputs.py), so these tests run without it."""
 import numpy as np
 import pytest
+
+from reference_outputs import Reference, assert_same
 
 
 @pytest.fixture(scope="module")
 def ref(oracle):
-    if not oracle.ref_lsd_available():
-        pytest.skip("oracle/_ref/liblsd_ref.so not built (no /root/reference on this machine)")
-    return oracle
+    r = Reference(oracle, __name__)
+    yield r
+    r.save()
 
 
 def _same(ref, img):
     got = ref.lsd_detect(img, 15.0)["raw_lines"]
     want = ref.ref_lsd_detect(img)
     assert got.shape == want.shape
-    np.testing.assert_array_equal(got, want)
+    assert_same(got, want)
     return len(want)
 
 
